@@ -5,14 +5,16 @@ One "step" = one pass of the hot path over one batch of synthetic input: control
 prefill -> N-1 KV-cache decode steps with CFG + top-k sampling -> VQGAN decode of the token grids, i.e. exactly
 `generate()` + `decode_code()` of autoregressive/sample/sample_t2i.py:163-176, through this repo's drop-in modules.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|4t]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|4t] [--dump-outputs DIR]
 
   --config 2  (default) BASELINE.json configs[1]: XL + DINOv2-small canny, 512x512, batch 8 per GPU
   --config 3  configs[2]: XL + DINOv2-base depth, 512x512, batch 8 per GPU (64 images on 8 GPUs)
   --config 4  configs[3]: XL canny_MR 768x512 (W x H, 1536 tokens, RoPE table side 48), batch 4; 4t = 512x768 (tall)
 
 N > 1 is launched with torchrun (one rank per GPU); every rank generates its own `--batch` images (weak scaling)
-and the int32 token grids are all-gathered once over NCCL.  `--impl reference` times the CPU restatement of the
+and the int32 token grids are all-gathered once over NCCL.  `--dump-outputs DIR` saves what the last timed step returned to its
+caller (rank 0's token grids and decoded images); inputs, weights and sampling seeds depend only on the arguments, so two builds
+run with the same arguments can be compared output for output.  `--impl reference` times the CPU restatement of the
 reference path (oracle/, kind "port": the reference is Python and /root/reference does not exist on the GPU box)
 on the host cores.
 """
@@ -29,6 +31,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # no __pycache__ beside the sources: bench.py leaves the tree as build() left it
 
 import torch
 
@@ -52,7 +55,13 @@ def parse():
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the reference PyTorch-eager measurement on the GPU (gpu_eager_baseline)")
     ap.add_argument("--ref-compile", action="store_true", help="also time the reference's torch.compile(mode='reduce-overhead') path (minutes of compile)")
     ap.add_argument("--config", default="2", choices=["2", "3", "4", "4t"], help="BASELINE.json config preset (sets size/batch/adapter/condition)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the token grids and images of the last timed step (rank 0) to DIR/<name>.npy as float32")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to the timed GPU path (--impl ours)")
     if a.config == "3":
         a.adapter_size, a.condition_type = "base", "depth"
     elif a.config in ("4", "4t"):
@@ -177,14 +186,14 @@ def cpu_reference_images_per_sec(args, n_decode_steps=32, repeats=3, threads=Non
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# Reference GPU baseline (SURVEY.md 8(d)): the UNMODIFIED reference modules from baseline/_ref (scripts/install_ref.sh) run
+# Reference GPU baseline (SURVEY.md 8(d)): the UNMODIFIED reference modules from oracle/_ref (oracle/install_ref.sh, run by build()) run
 # eagerly on this GPU through the reference's own generate() + decode_code() (sample_t2i.py:163-176).  Warm-up 1 short call,
 # then the median of 3 full calls, CUDA events.  The north_star target (>= 4x) is defined against this number.
 # ---------------------------------------------------------------------------------------------------------------
 def gpu_eager_reference(args, dev, cond_d, masks_d, cmap_d, n_calls=3, compile_too=False):
-    ref_root = os.path.join(ROOT, "baseline", "_ref")
+    ref_root = os.path.join(ROOT, "oracle", "_ref")
     if not os.path.isdir(os.path.join(ref_root, "autoregressive", "models")):
-        return {"unavailable": "baseline/_ref missing: run scripts/install_ref.sh in the build container"}
+        return {"unavailable": "oracle/_ref missing: build() makes it where a checkout of the reference exists (oracle/install_ref.sh)"}
     import contextlib, io, tempfile, warnings
     warnings.filterwarnings("ignore")
     H_img, W_img, gh, gw = _dims(args)
@@ -232,7 +241,7 @@ def gpu_eager_reference(args, dev, cond_d, masks_d, cmap_d, n_calls=3, compile_t
         ms = sorted(call(N, ref_generate) for _ in range(n_calls))
         med = ms[len(ms) // 2]
         out = {"value": B / (med * 1e-3), "unit": "images/s", "ms_per_batch": med, "ms_per_decode_step": med / N, "calls": n_calls,
-               "spread": (ms[-1] - ms[0]) / med, "impl": "reference modules (baseline/_ref, unmodified) PyTorch eager, bf16 AR + fp32 VQ, "
+               "spread": (ms[-1] - ms[0]) / med, "impl": "reference modules (oracle/_ref, unmodified) PyTorch eager, bf16 AR + fp32 VQ, "
                f"torch {torch.__version__}", "config": f"{args.model} {W_img}x{H_img} batch {B} cfg {args.cfg_scale} top-k {args.top_k}"}
         if compile_too:
             try:
@@ -267,15 +276,36 @@ def _config_block(args, world):
             "sampling": {"cfg_scale": args.cfg_scale, "top_k": args.top_k, "temperature": 1.0, "top_p": 1.0}}
 
 
+DUMP_BYTES = 64_000_000        # cap on everything --dump-outputs writes, .npy headers included (64 MB, decimal)
+NPY_HEADER = 128               # bytes np.save puts in front of a 1- to 4-d float array
+
+
+def dump_outputs(path, arrays):
+    """One float32 DIR/<name>.npy per output, smallest first; each output may use an even share of what DUMP_BYTES has left, so the
+    budget the small ones leave unused goes to the larger.  An output larger than its share is cut to a fixed seeded sample of its
+    elements, whose flat indices go to DIR/<name>_index.npy (float64: 12 bytes per sampled element with the value)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel())):
+        share = left // (len(arrays) - i)
+        a = t.float().numpy()
+        if a.nbytes + NPY_HEADER > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, (share - 2 * NPY_HEADER) // 12, replace=False))
+            np.save(os.path.join(path, name + "_index.npy"), idx.astype(np.float64))
+            left -= idx.size * 8 + NPY_HEADER
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes + NPY_HEADER
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     # one step = the bounded CPU sample of the workload (cpu_reference_images_per_sec: the full batch, prefill + 3 x 32 decode steps,
-    # about a minute of host work); the whole arm is capped at ~4 minutes: one untimed sample if requested, then up to `steps` timed ones
+    # about a minute of host work): one untimed sample if warm-up is requested, then exactly `steps` timed ones
     vals = []
-    t_start = time.perf_counter()
-    budget = 240.0
     n_warm = 0
     if args.warmup > 0:
         cpu_reference_images_per_sec(args, n_decode_steps=4, repeats=1)        # touches every weight page once
@@ -283,8 +313,6 @@ def run_reference(args):
     while len(vals) < args.steps:
         ips, cores, sample = cpu_reference_images_per_sec(args)
         vals.append(ips)
-        if time.perf_counter() - t_start > budget:
-            break
     v = sorted(vals)[len(vals) // 2]
     line = {"metric": "images/sec", "value": v, "unit": "images/s", "n_gpus": args.gpus, "steps": len(vals), "warmup": n_warm,
             "ms_per_step": 1000.0 * args.batch / v, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -359,13 +387,13 @@ def run_ours(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(n_steps):
-            one_step(first_idx + i, host_io)
+            last = one_step(first_idx + i, host_io)
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms)
+        return float(ms), last
 
     for i in range(args.warmup):
         one_step(i, False)
@@ -374,9 +402,10 @@ def run_ours(args):
     if rank == 0:
         clocks.start()
     lib.car_launch_count(1)
-    ms = timed(args.steps, False, args.warmup)
+    ms, (last_toks, last_img) = timed(args.steps, False, args.warmup)
     launches = int(lib.car_launch_count(0))
-    ms_e2e = timed(args.steps, True, args.warmup + args.steps)
+    outputs = {"tokens": last_toks.cpu(), "images": last_img.cpu()} if args.dump_outputs and rank == 0 else None
+    ms_e2e, _ = timed(args.steps, True, args.warmup + args.steps)
     # decode-loop roofline: time the device-side decode loop alone (prefill excluded) with CUDA events on the stream
     # the kernels are launched on (torch's current stream is the stream handed to the library)
     st = gpt._car_state
@@ -458,6 +487,8 @@ def run_ours(args):
     if not args.no_cpu_baseline and world == 1:
         v, cores, sample = cpu_reference_images_per_sec(args, n_decode_steps=16, repeats=3)
         line["cpu_baseline"] = {"value": v, "unit": "images/s", "cores": cores, "kind": "port", "sample": sample}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,5 +1,5 @@
 """The reference's own training step on this GPU, for comparison with scripts/bench_train.py: the UNMODIFIED reference modules
-(baseline/_ref, scripts/install_ref.sh) driven like autoregressive/train/train_c2i_canny.py:190-211 — fp32 parameters,
+(oracle/_ref, oracle/install_ref.sh) driven like autoregressive/train/train_c2i_canny.py:190-211 — fp32 parameters,
 `torch.autocast(bf16)`, `model(cond_idx, idx, targets, condition)`, `loss.backward()`, `torch.optim.AdamW(fused=True).step()` —
 on the BASELINE.json config-5 shape (LlamaGen-L c2i 256 x 256, DINOv2-small canny adapter, 32 images per GPU), PyTorch eager.
 --freeze-adapter stops the gradient at the control tokens, which is where controlar_b200's backward stops (like for like);
@@ -30,8 +30,8 @@ def main():
     args = ap.parse_args()
     warnings.filterwarnings("ignore")
     dev = torch.device(args.device)
-    ref_root = os.path.join(ROOT, "baseline", "_ref")
-    assert os.path.isdir(os.path.join(ref_root, "autoregressive", "models")), "baseline/_ref missing: run scripts/install_ref.sh"
+    ref_root = os.path.join(ROOT, "oracle", "_ref")
+    assert os.path.isdir(os.path.join(ref_root, "autoregressive", "models")), "oracle/_ref missing: run oracle/install_ref.sh <reference checkout>"
     from transformers import Dinov2Config, Dinov2Model
     n = (args.image_size // 16) ** 2
     old_cwd = os.getcwd()
@@ -93,7 +93,7 @@ def main():
             rows.append((*t, float(loss.detach())))
     med = lambda i: sorted(r[i] for r in rows)[len(rows) // 2]
     total = med(0) + med(1) + med(2)
-    print(json.dumps({"impl": "reference modules (baseline/_ref, unmodified), PyTorch eager, bf16 autocast, torch " + torch.__version__,
+    print(json.dumps({"impl": "reference modules (oracle/_ref, unmodified), PyTorch eager, bf16 autocast, torch " + torch.__version__,
                       "workload": f"{args.model} c2i {args.image_size}^2 training step, batch {B} per GPU", "adapter_frozen": args.freeze_adapter,
                       "forward_loss_ms": med(0), "backward_ms": med(1), "adamw_ms": med(2), "images_per_s": 1000.0 * B / total,
                       "loss_first": rows[0][3], "loss_last": rows[-1][3], "steps": args.steps, "warmup": args.warmup}))

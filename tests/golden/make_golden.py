@@ -510,6 +510,83 @@ def train_case(name: str, spec: GPTSpec, B: int, H: int, W: int, autocast, use_m
     print(name, "loss %.6f" % float(loss), "drop", seen["drop_ids"].tolist(), "grads", len(grads), flush=True)
 
 
+def gptpy_train_case(n_cols: int = 512):
+    """The LEGACY class gpt.py in train mode (fp32, the configuration its train_c2i_canny.py uses: cls_token_num = 1,
+    condition_token_num = 0) -> the CFG drop decision, the adapter output, the loss and the logits at a fixed seeded set of
+    `n_cols` vocabulary columns (all rows).  tests/test_train_oracle_golden.py pins oracle/train_oracle.py against it."""
+    from autoregressive.models.gpt import Transformer, ModelArgs
+    from oracle.weights import vit_shapes, _fill
+    from oracle.inputs import code_inputs
+    seed, B, H, W = 0, 4, 64, 64
+    spec = GPTSpec(**SMALL, cls_token_num=1, block_size=(H // 16) * (W // 16), model_type="c2i")
+    with fake_vit_cwd(2), contextlib.redirect_stdout(io.StringIO()):
+        m = Transformer(ModelArgs(dim=spec.dim, n_layer=spec.n_layer, n_head=spec.n_head, multiple_of=spec.multiple_of,
+                                  vocab_size=spec.vocab_size, cls_token_num=1, block_size=spec.block_size, num_classes=spec.num_classes,
+                                  model_type="c2i", condition_token_num=0, image_size=H, token_dropout_p=0.0, resid_dropout_p=0.0,
+                                  ffn_dropout_p=0.0, class_dropout_prob=0.5))
+    full = make_gpt_state_dict(spec, seed, with_adapter=False)
+    full.update(_fill(vit_shapes(384, layers=2, prefix="adapter.model."), seed, 0.02))
+    full["condition_norm.weight"] = torch.ones(spec.dim)
+    m.load_state_dict(full, strict=True)
+    m = m.float().train()
+    cond = class_inputs(spec.num_classes, B, seed + 1)
+    cmap = control_map(B, H, W, seed + 2, "canny", torch.float32)
+    z = code_inputs(spec.vocab_size, B, spec.block_size, seed + 4)
+    seen = {}
+    orig_drop = m.cls_embedding.token_drop
+
+    def spy_drop(*a, **k):
+        out = orig_drop(*a, **k)
+        seen["drop_ids"] = out[1].clone()
+        return out
+    m.cls_embedding.token_drop = spy_drop
+    hook = m.adapter.register_forward_hook(lambda mod, inp, out: seen.__setitem__("feat", out.detach().clone()))
+    torch.manual_seed(1)
+    with math_sdpa():
+        logits, loss = m(cond_idx=cond, idx=z[:, :-1], targets=z, condition=cmap)
+    hook.remove()
+    cols = torch.randperm(spec.vocab_size, generator=torch.Generator().manual_seed(seed + 13))[:n_cols].sort().values
+    out = {"header": header(), "spec": spec.__dict__, "seed": seed, "B": B, "H": H, "W": W, "sdpa": "math",
+           "class": "autoregressive/models/gpt.py Transformer (legacy c2i class), ViT layers = 2, train mode, fp32",
+           "dropout": "token/resid/ffn p = 0; class_dropout_prob = 0.5, torch.manual_seed(1)",
+           "inputs": "oracle.inputs: class_inputs(seed+1), control_map(seed+2), code_inputs(seed+4)",
+           "drop_ids": seen["drop_ids"], "feat": seen["feat"], "loss": loss.detach().clone(),
+           "logits_shape": tuple(logits.shape), "cols": cols, "logits_cols": logits.detach()[..., cols].float().clone()}
+    torch.save(out, os.path.join(OUT, "train_c2i_gptpy_fp32.pt"))
+    print("gptpy train loss %.6f" % float(loss), "drop", seen["drop_ids"].tolist(), "feat", tuple(seen["feat"].shape), flush=True)
+
+
+def reference_surface_case():
+    """The parts of the reference's public surface the drop-in must reproduce: ModelArgs fields and defaults, the parameter
+    lists of generate() / the sampling helpers / Transformer.forward, and the .py files of the packages the drop-in tree is put
+    in front of (none of them has an __init__.py: all are namespace packages) -> reference_surface.json."""
+    import dataclasses
+    import inspect
+    import json
+    import autoregressive.models.gpt_t2i as t2i
+    import autoregressive.models.gpt as gpt
+    import autoregressive.models.generate as gen
+
+    def params(fn):
+        return list(inspect.signature(fn).parameters)
+    tree = []
+    for d in ("autoregressive", "autoregressive/models", "autoregressive/serve", "tokenizer", "tokenizer/tokenizer_image",
+              "condition", "utils", "dataset"):
+        tree += sorted(f"{d}/{f}" for f in os.listdir(os.path.join(REF, d)) if f.endswith(".py"))
+    out = {"generator": "tests/golden/make_golden.py reference_surface",
+           "model_args": {name: {f.name: f.default for f in dataclasses.fields(mod.ModelArgs)}
+                          for name, mod in (("gpt_t2i", t2i), ("gpt", gpt))},
+           "signatures": {"generate": params(gen.generate), "sample": params(gen.sample),
+                          "top_k_top_p_filtering": params(gen.top_k_top_p_filtering), "logits_to_probs": params(gen.logits_to_probs),
+                          "gpt_t2i.Transformer.forward": params(t2i.Transformer.forward),
+                          "gpt.Transformer.forward": params(gpt.Transformer.forward)},
+           "tree": tree}
+    with open(os.path.join(OUT, "reference_surface.json"), "w") as fh:
+        json.dump(out, fh, indent=1)
+        fh.write("\n")
+    print("reference surface ok", len(tree), "files", flush=True)
+
+
 XL = dict(dim=1280, n_layer=36, n_head=20, vocab_size=16384)
 
 
@@ -628,6 +705,8 @@ CASES = {
     "hed": hed_case,
     "t5": t5_case,
     "c2i_gptpy_bf16": gptpy_case,
+    "train_c2i_gptpy_fp32": gptpy_train_case,
+    "reference_surface": reference_surface_case,
     "train_t2i_small_ac": lambda: train_case("train_t2i_small_ac", GPTSpec(**SMALL, cls_token_num=120, block_size=64, model_type="t2i"),
                                              B=3, H=128, W=128, autocast=torch.bfloat16, use_mask=True, valid=[1, 0, 1]),
     "train_t2i_small_fp32": lambda: train_case("train_t2i_small_fp32", GPTSpec(**SMALL, cls_token_num=120, block_size=64, model_type="t2i"),

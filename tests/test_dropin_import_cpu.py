@@ -1,13 +1,13 @@
 """Row b (drop-in boundary): the PYTHONPATH configuration INTEGRATION.md documents must make the reference's own import lines
 (autoregressive/sample/sample_t2i.py:15-19, sample_c2i.py:19) resolve to this repository's modules — checked in a fresh interpreter,
-from a foreign working directory.  With /root/reference present (build container) the modules this repository does NOT replace
-must still resolve to the reference tree."""
+from a foreign working directory.  Behind it, the modules this repository does NOT replace must still resolve to the reference
+tree: checked against a stand-in tree with the reference's package layout (tests/golden/reference_surface.json)."""
+import json
 import os
 import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 CODE = r"""
 import os, sys
@@ -43,8 +43,21 @@ def test_dropin_imports_resolve_to_this_repo(tmp_path):
     _run([], [], tmp_path)
 
 
+def _reference_tree(dst):
+    """Placeholder modules at the reference's .py paths, without __init__.py files like the reference: which directory a module
+    resolves from depends only on that layout."""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_surface.json")) as fh:
+        files = json.load(fh)["tree"]
+    for rel in files:
+        path = os.path.join(dst, *rel.split("/"))
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        with open(path, "w") as fh:
+            fh.write(f'"""Stand-in for the reference\'s {rel}."""\n')
+    return str(dst)
+
+
 def test_dropin_in_front_of_the_reference_tree(tmp_path):
-    import pytest
-    if not os.path.isdir(REF):
-        pytest.skip("no /root/reference on this box")
-    _run([REF], [REF], tmp_path)
+    ref = _reference_tree(tmp_path / "reference")
+    work = tmp_path / "work"
+    work.mkdir()
+    _run([ref], [ref], work)

@@ -1,27 +1,18 @@
 """CPU: the drop-in surface (SURVEY.md §8b) — constructor fields, function signatures, registry keys and state-dict keys of
 the product shells against the reference.  The state-dict key sets come from oracle/weights.py, which
-tests/golden/make_golden.py asserts equal to the reference modules' own ``state_dict()``; where /root/reference is present
-(the build container) the dataclass fields and signatures are compared with the reference source directly."""
+tests/golden/make_golden.py asserts equal to the reference modules' own ``state_dict()``; the dataclass fields and signatures
+are compared with the reference's as recorded from its source by make_golden.py (tests/golden/reference_surface.json)."""
 import dataclasses
 import inspect
+import json
 import os
-import sys
 
-import pytest
 import torch
 
 from oracle.weights import GPTSpec, gpt_shapes, vit_shapes, vq_shapes
 
-REF = "/root/reference"
-
-
-def _ref_module(name):
-    if not os.path.isdir(REF):
-        pytest.skip("reference tree not available on this machine")
-    if REF not in sys.path:
-        sys.path.append(REF)           # after the repo: `oracle`, `tests`, `controlar_b200` keep resolving to this repo
-    import importlib
-    return importlib.import_module(name)
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_surface.json")) as _fh:
+    REF = json.load(_fh)
 
 
 def test_state_dict_keys_t2i_and_c2i():
@@ -68,25 +59,23 @@ def test_model_args_fields_match_reference():
         "controlar_b200.autoregressive.models.gpt_t2i", fromlist=["ModelArgs"]).ModelArgs)}
     ours_gpt = {f.name: f.default for f in dataclasses.fields(__import__(
         "controlar_b200.autoregressive.models.gpt", fromlist=["ModelArgs"]).ModelArgs)}
-    ref_t2i = {f.name: f.default for f in dataclasses.fields(_ref_module("autoregressive.models.gpt_t2i").ModelArgs)}
-    ref_gpt = {f.name: f.default for f in dataclasses.fields(_ref_module("autoregressive.models.gpt").ModelArgs)}
-    assert ours_t2i == ref_t2i
-    assert ours_gpt == ref_gpt
+    assert ours_t2i == REF["model_args"]["gpt_t2i"]
+    assert ours_gpt == REF["model_args"]["gpt"]
 
 
 def test_generate_and_forward_signatures_cover_the_reference():
     from controlar_b200.autoregressive.models import generate as og, gpt_t2i as ot, gpt as ol
-    rg = _ref_module("autoregressive.models.generate")
-    ref_params = list(inspect.signature(rg.generate).parameters)
+    sig = REF["signatures"]
+    ref_params = sig["generate"]
     our_params = list(inspect.signature(og.generate).parameters)
     assert [p for p in our_params if p in ref_params] == ref_params                       # same names, same order
     assert set(our_params) - set(ref_params) <= {"noise", "seed"}                         # keyword-only extras
     for name in ("sample", "top_k_top_p_filtering", "logits_to_probs"):
-        rp, op = inspect.signature(getattr(rg, name)).parameters, inspect.signature(getattr(og, name)).parameters
+        rp, op = sig[name], inspect.signature(getattr(og, name)).parameters
         assert list(rp)[:2] == list(op)[:2], name
-    rf = list(inspect.signature(_ref_module("autoregressive.models.gpt_t2i").Transformer.forward).parameters)
+    rf = sig["gpt_t2i.Transformer.forward"]
     assert list(inspect.signature(ot.Transformer.forward).parameters) == rf
-    rl = list(inspect.signature(_ref_module("autoregressive.models.gpt").Transformer.forward).parameters)
+    rl = sig["gpt.Transformer.forward"]
     assert list(inspect.signature(ol.Transformer.forward).parameters)[:len(rl)] == rl     # + control_strength (must stay 1)
 
 

@@ -122,46 +122,16 @@ def test_legacy_gptpy_train_branch_is_the_same_arithmetic():
     (gpt.py:410-421,440-449).  With the only configuration its scripts use (cls_token_num = 1, condition_token_num = 0) it is the
     gpt_t2i branch: control tokens added to every row, logits from row 0 on.  Pinned here by running the reference's gpt.py in
     train mode (fp32) against the oracle on the same weights — which is why controlar_b200's gpt.py shell inherits the training
-    forward / backward of gpt_t2i unchanged.  Needs /root/reference (build container); skipped elsewhere."""
-    import contextlib
-    import io
-    import os
-    if not os.path.isdir("/root/reference/autoregressive/models"):
-        pytest.skip("reference sources not present")
-    from tests.golden import make_golden as mg
-    from autoregressive.models.gpt import Transformer as RefLegacy, ModelArgs as RefArgs      # the reference's legacy class
-    from oracle.weights import vit_shapes, _fill
-    from oracle.inputs import control_map
-    seed, B, H, W = 0, 4, 64, 64
-    spec = GPTSpec(**mg.SMALL, cls_token_num=1, block_size=(H // 16) * (W // 16), model_type="c2i")
-    with mg.fake_vit_cwd(2), contextlib.redirect_stdout(io.StringIO()):
-        m = RefLegacy(RefArgs(dim=spec.dim, n_layer=spec.n_layer, n_head=spec.n_head, multiple_of=spec.multiple_of, vocab_size=spec.vocab_size,
-                              cls_token_num=1, block_size=spec.block_size, num_classes=spec.num_classes, model_type="c2i",
-                              condition_token_num=0, image_size=H, token_dropout_p=0.0, resid_dropout_p=0.0, ffn_dropout_p=0.0,
-                              class_dropout_prob=0.5))
+    forward / backward of gpt_t2i unchanged.  The reference's side (its CFG drop decision, adapter output, loss and logits at 512
+    seeded vocabulary columns) is stored by tests/golden/make_golden.py::gptpy_train_case."""
+    g = load_golden("train_c2i_gptpy_fp32")
+    spec = GPTSpec(**g["spec"])
+    seed, B = g["seed"], g["B"]
     sd = make_gpt_state_dict(spec, seed, with_adapter=False)
-    full = dict(sd)
-    full.update(_fill(vit_shapes(384, layers=2, prefix="adapter.model."), seed, 0.02))
-    full["condition_norm.weight"] = torch.ones(spec.dim)
-    m.load_state_dict(full, strict=True)
-    m = m.float().train()
     cond = class_inputs(spec.num_classes, B, seed + 1)
-    cmap = control_map(B, H, W, seed + 2, "canny", torch.float32)
     z = code_inputs(spec.vocab_size, B, spec.block_size, seed + 4)
-    seen = {}
-    orig_drop = m.cls_embedding.token_drop
-
-    def spy_drop(*a, **k):
-        out = orig_drop(*a, **k)
-        seen["drop_ids"] = out[1].clone()
-        return out
-    m.cls_embedding.token_drop = spy_drop
-    hook = m.adapter.register_forward_hook(lambda mod, inp, out: seen.__setitem__("feat", out.detach().clone()))
-    torch.manual_seed(1)
-    with torch.no_grad(), mg.math_sdpa():
-        logits, loss = m(cond_idx=cond, idx=z[:, :-1], targets=z, condition=cmap)
-    hook.remove()
-    assert seen["drop_ids"].any() and not seen["drop_ids"].all()
+    drop_ids, feat, cols, logits, loss = g["drop_ids"], g["feat"], g["cols"], g["logits_cols"], g["loss"]
+    assert drop_ids.any() and not drop_ids.all()
     # one difference: gpt.py's ConditionEmbedder.token_drop gives dropped samples literal zeros (gpt.py:118-119), gpt_t2i's gives
     # them the `uncond_embedding` buffer (gpt_t2i.py:120) — identical for released checkpoints (the buffer is zero), not for the
     # procedural weights used here.  controlar_b200's gpt.py shell therefore passes no buffer (cond_uncond = NULL => zeros).
@@ -169,9 +139,9 @@ def test_legacy_gptpy_train_branch_is_the_same_arithmetic():
     sd0["condition_mlp.uncond_embedding"] = torch.zeros_like(sd["condition_mlp.uncond_embedding"])
     orc = TrainOracle(spec, sd0, None)
     with torch.no_grad():
-        lo, ls = orc.forward(z[:, :-1], cond, seen["feat"], seen["drop_ids"], None, z, None)
-        lb, _ = TrainOracle(spec, sd, None).forward(z[:, :-1], cond, seen["feat"], seen["drop_ids"], None, z, None)
-    assert lo.shape == logits.shape
-    assert rel_l2(lo, logits.float()) < 5e-6
+        lo, ls = orc.forward(z[:, :-1], cond, feat, drop_ids, None, z, None)
+        lb, _ = TrainOracle(spec, sd, None).forward(z[:, :-1], cond, feat, drop_ids, None, z, None)
+    assert tuple(lo.shape) == tuple(g["logits_shape"])
+    assert rel_l2(lo[..., cols], logits) < 5e-6
     assert abs(float(ls) - float(loss)) < 5e-6 * float(loss)
-    assert rel_l2(lb, logits.float()) > 1e-3          # with the buffer's rows instead of zeros the result is visibly different
+    assert rel_l2(lb[..., cols], logits) > 1e-3       # with the buffer's rows instead of zeros the result is visibly different
